@@ -3,6 +3,15 @@
 
   python bench.py --gpus N --steps K --warmup W            # our CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path
+  python bench.py --gpus 1 --steps K --dump-outputs DIR    # + [Ψ; acc] of the last timed step as .npy
+
+Every timed region runs exactly K steps (the e2e region too, unless --e2e-steps says otherwise).
+The inputs are drawn from fixed seeds, so two runs with the same arguments sweep the same pools
+at the same ν.  The outputs agree to summation-order noise, not bit for bit: the kernel sizes
+each CTA's pool range from measured CTA speed (option `balance`), so the fp64 parts of the sums
+(acc, pools outside the fixed-point slice) are added in a timing-dependent order; on a B200,
+two runs of the default workload differed by at most 2e-12 relative in Ψ.  The run writes
+nothing into the source tree.
 
 A "step" is ONE dual-gradient sweep: find_arb! over every pool at the current
 ν plus the Ψ / acc folds (src/router.jl:38-42, 79-83, 98-100) -- exactly what
@@ -35,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ from the imports below
 
 METRIC = "find_arb_pools_per_sec_per_dual_gradient_sweep"
 UNIT = "pools/s"
@@ -63,12 +73,23 @@ def parse_args():
     ap.add_argument("--nu", choices=["near", "wide", "ones"], default="near")
     ap.add_argument("--exact", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="0 = same as --steps (capped)")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="0 = same as --steps")
+    ap.add_argument("--sustained-ms", type=float, default=0.0,
+                    help="when the K timed steps take less than this many ms, also time a longer region of the "
+                         "same steps (`sustained`, clocks sampled under load); 0 = off, so that only K steps "
+                         "are timed per region")
     ap.add_argument("--no-flush", action="store_true", help="small workloads: L2-warm timing only")
     ap.add_argument("--verify", type=int, default=1, help="N > 1: check the reduced [Psi; acc] (outside the timed regions)")
     ap.add_argument("--opt", action="append", default=[], help="library option key=value (measurement)")
     ap.add_argument("--strong", type=int, default=1, help="N > 1 (weak): also time the same total pool count split over the ranks")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed, the float64 arrays a caller of the sweep "
+                         "receives, to DIR/psi.npy and DIR/acc.npy (inputs are seeded: two builds can be "
+                         "compared output for output, within summation-order noise)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm times a machine-dependent sample)")
+    return args
 
 
 def make_shard(workload, rank, world, scaling):
@@ -338,13 +359,15 @@ def run_ours(args):
         flush_buf.zero_()
         flush_rd.sum()
 
+    last_out = [d_psi.data_ptr()]  # device address of the [Ψ; acc] the last step wrote
+
     def make_step(p):
         def step():
             if exchange == "nccl":  # NCCL needs the partial in a torch tensor
                 p.sweep_device(d_nu.data_ptr(), d_psi.data_ptr(), False, sptr)
                 dist.all_reduce(d_psi)
             else:  # zero-copy: [Ψ; acc] stays in the context's device buffer
-                p.sweep_device_view(d_nu.data_ptr(), False, sptr)
+                last_out[0] = p.sweep_device_view(d_nu.data_ptr(), False, sptr)
         return step
 
     step = make_step(pools)
@@ -425,16 +448,18 @@ def run_ours(args):
         sampler.start()
         ms_total = timed_region(args.steps, flush=flushed)
         launches = pools.launch_count - l0
+        # the result of the last timed step, before any later sweep overwrites the context's buffer
+        outputs = _view(torch, last_out[0], n + 1, dev).clone() if args.dump_outputs and rank == 0 else None
         extra["host_enqueue_us_per_step"] = host_enqueue_us[0]
-        # a driver-sized K can be a millisecond of GPU time: also a region of >= 50 ms of the
-        # same steps (`sustained`), so that the clocks are sampled under load
+        # a small K can be a millisecond of GPU time: on request, also a region of at least
+        # --sustained-ms of the same steps (`sustained`), so that the clocks are sampled under load
         ms_dec = ms_total
         if world > 1:  # every rank must take the same branch and launch the same number of sweeps
             t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms_dec = t.item()
-        if ms_dec < 50.0 and not flushed:
-            k2 = int(min(50_000, max(args.steps, np.ceil(60.0 * args.steps / max(ms_dec, 1e-3)))))
+        if ms_dec < args.sustained_ms and not flushed:
+            k2 = int(min(50_000, max(args.steps, np.ceil(1.2 * args.sustained_ms * args.steps / max(ms_dec, 1e-3)))))
             ms2 = timed_region(k2)
             extra["sustained"] = {"steps": k2, "ms_per_step": ms2 / k2}
         sampler.stop()
@@ -453,7 +478,7 @@ def run_ours(args):
         pools.set_option("profile", 0)
 
         # ---- e2e: public C-ABI call with pinned host buffers, copies inside ----
-        e2e_steps = args.e2e_steps or min(args.steps, 2000)
+        e2e_steps = args.e2e_steps or args.steps
         h_nu = torch.from_numpy(nu_host).pin_memory()
         h_out = torch.zeros(n + 1, dtype=torch.float64).pin_memory()  # [psi ; acc] contiguous
         h_psi, h_acc = h_out[:n], h_out[n:]
@@ -552,10 +577,20 @@ def run_ours(args):
         }
         line["ingest"] = ingest
         line.update(extra)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs.cpu().numpy(), n)
         emit(line)
     pools.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, psi_acc, n):
+    """[Ψ; acc] of one sweep (float64, n_tokens + 1: at most 400 KB for the workloads above) as
+    DIR/psi.npy [n_tokens] and DIR/acc.npy [1]."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "psi.npy"), np.ascontiguousarray(psi_acc[:n], dtype=np.float64))
+    np.save(os.path.join(out_dir, "acc.npy"), np.ascontiguousarray(psi_acc[n:], dtype=np.float64))
 
 
 def _view(torch, ptr, count, dev):
@@ -679,7 +714,7 @@ def strong_scaling_run(torch, dist, cr, args, pools_weak, make_step, timed_regio
     if args.protocol > 0:
         ps.set_option("exchange_protocol", args.protocol)
     fn = make_step(ps)
-    steps = max(args.steps, 200)
+    steps = args.steps
     for _ in range(10):
         fn()
     ms = timed_region(steps, fn)

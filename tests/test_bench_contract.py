@@ -1,12 +1,13 @@
 """bench.py pieces that run without a GPU: the `roofline` object arithmetic and
-the reference arm (the CPU port timed on the host cores), which must print the
-contract's one JSON line."""
+the reference arm (the CPU port timed on the host cores), which must print
+one JSON line; on a GPU, the step count and `--dump-outputs`."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -73,3 +74,31 @@ def test_reference_arm_prints_contract_line():
     assert r["metric"] and r["unit"] == "pools/s" and r["value"] > 0 and r["steps"] == 2
     assert r["cpu_baseline"]["kind"] == "port" and r["cpu_baseline"]["cores"] >= 1
     assert r["e2e"]["value"] == r["value"] and r["e2e"]["h2d_bytes_per_step"] == 0
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_timed_sweep(oracle, synth, tmp_path):
+    """`--steps K` times K sweeps (one launch each), and `--dump-outputs` writes the [Ψ; acc]
+    the last of them computed: the CPU oracle's fold of the same seeded pools at the same ν."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "7", "--warmup", "2",
+                          "--workload", "config2_100k_product_1k_tokens", "--no-cpu-baseline",
+                          "--dump-outputs", str(tmp_path / "out")],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    r = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][0])
+    assert r["steps"] == 7 and r["gpu_launches"] == 7 and r["e2e"]["steps"] == 7 and "sustained" not in r
+    psi, acc = np.load(tmp_path / "out" / "psi.npy"), np.load(tmp_path / "out" / "acc.npy")
+    n = 1_000
+    assert psi.dtype == np.float64 and psi.shape == (n,) and acc.shape == (1,)
+    R, g, Ai = synth.product_pools(100_000, n, seed=1234)
+    v = synth.dual_prices(n, "near")
+    D, L = oracle.sweep_product(R, g, Ai, v, threads=8)
+    accx, Gx, absG = oracle.fold_compensated(Ai, D, L, v, n)
+    slack, S, deg = np.zeros(n), np.zeros(n), np.zeros(n)  # economized math + fixed-point slice quantum,
+    for side in (0, 1):                                    # as bench.verify_reduction bounds them
+        np.add.at(slack, Ai[:, side] - 1, 32 * np.finfo(float).eps * (R[:, 0] + R[:, 1]) / g)
+        np.add.at(S, Ai[:, side] - 1, R[:, side])
+        np.add.at(deg, Ai[:, side] - 1, 1.0)
+    slack += deg * S * 2.0 ** -53
+    assert np.all(np.abs(psi - Gx.astype(np.float64)) <= 1e-12 * absG + slack)
+    assert abs(acc[0] - float(accx)) <= 1e-12 * float(np.sum(absG * v)) + float(np.sum(slack * v))
